@@ -19,7 +19,11 @@ A step = one pass of the hot path over one frame of synthetic input.
   python bench.py --gpus N --steps K --warmup W           # CUDA arm
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port, all host threads)
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  With --dump-outputs DIR, rank 0 also writes what the last timed step computed as
+DIR/<name>.npy (finite float32 / float64), a fixed seeded sample of DUMP_PIXELS pixels per image, so that two
+builds can be compared output for output:
+  frame2d_distance, _kind, _fill_depth, _inside   N = 1: the 2D frame's RawDistancePixel words, unpacked
+  volume3d_depth, _normal      the 3D frame's GeometryPixel depth and normal (N = 1 unless --no-volume, and N > 1)
 """
 from __future__ import annotations
 
@@ -45,11 +49,51 @@ ALGO_BYTES_PER_PIXEL_3D = 16   # one GeometryPixel written per pixel
 T0 = 128
 WORKLOAD_2D = f"models/{MODEL} 2D render {SIZE}x{SIZE}, tile sizes [128,32,8], identity camera"
 WORKLOAD_3D = f"models/{MODEL} 3D render {SIZE}^3, tile sizes [128,64,32,16,8], identity camera"
+# 2^20 of the 2^24 pixels of a frame: the four 2D arrays (16 MiB) and the 3D depth + normals (20 MiB) stay under 64 MB
+DUMP_PIXELS = 1 << 20
+DUMP_SEED = 0
 
 
 def model_text():
     with open(os.path.join(ROOT, "models", MODEL)) as f:
         return f.read()
+
+
+def sample_pixels(img):
+    """The same DUMP_PIXELS pixels (seeded, in row-major order) of an [H, W, ...] image, numpy or CUDA tensor."""
+    n = img.shape[0] * img.shape[1]
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(DUMP_PIXELS, n), replace=False))
+    flat = img.reshape((n,) + tuple(img.shape[2:]))
+    if isinstance(img, np.ndarray):
+        return flat[idx]
+    import torch
+    return flat[torch.from_numpy(idx).to(img.device)].cpu().numpy()
+
+
+def frame2d_outputs(img):
+    """RawDistancePixel words unpacked into finite arrays (the words themselves NaN-box the fill pixels): kind 0 =
+    distance value, 1 = fill, 2 / 3 / 4 = NaN / +inf / -inf distance; the fill's recursion depth; inside as 0 / 1."""
+    from fidget_b200.shape import pixel_inside
+    px = sample_pixels(img)
+    bits = px.view(np.uint32)
+    fill = np.isnan(px) & ((bits & np.uint32(0xFF << 9)) == np.uint32(0xF6 << 9))   # RawDistancePixel::KEY
+    kind = np.select([fill, np.isnan(px), px == np.inf, px == -np.inf], [1, 2, 3, 4], 0)
+    return {"frame2d_distance": np.where(kind == 0, px, 0).astype(np.float32),
+            "frame2d_kind": kind.astype(np.float32),
+            "frame2d_fill_depth": np.where(fill, (bits >> 1) & 0xFF, 0).astype(np.float32),
+            "frame2d_inside": pixel_inside(px).astype(np.float32)}
+
+
+def volume3d_outputs(img):
+    from fidget_b200.shape import GEOMETRY_PIXEL
+    px = np.ascontiguousarray(sample_pixels(img)).view(GEOMETRY_PIXEL).reshape(-1)   # [n, 4] float32 -> n pixels
+    return {"volume3d_depth": px["depth"].astype(np.float64), "volume3d_normal": px["normal"]}
+
+
+def dump_outputs(directory, outputs):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -193,8 +237,10 @@ def run_reference(args):
             orc.render2d(t, SIZE, SIZE, threads=threads)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            orc.render2d(t, SIZE, SIZE, threads=threads)
+            img, _ = orc.render2d(t, SIZE, SIZE, threads=threads)
         dt = (time.perf_counter() - t0) / args.steps
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, frame2d_outputs(img))
         v = SIZE * SIZE / dt / 1e6
         metric = METRIC
         workload = WORKLOAD_2D
@@ -202,7 +248,7 @@ def run_reference(args):
                   "built here (no rustc), so this is the C++ oracle port of VmShape + fidget-raster::pixel::render")
     else:
         # same workload as the CUDA arm at N > 1; a step is a bounded sample (1/4 of the root-tile columns)
-        steps = min(args.steps, 8)
+        steps = args.steps
         cpu_volume_sample(orc, t, threads)
         t0 = time.perf_counter()
         vox = 0
@@ -261,8 +307,14 @@ def main():
     ap.add_argument("--impl", default="cuda")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-volume", action="store_true", help="N = 1: skip the 4096^3 strong-scaling base")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs and args.gpus > 1:
+            ap.error("--dump-outputs: the reference arm at N > 1 times a sample of the volume, not a whole frame")
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
 
@@ -301,16 +353,21 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
+    outputs = {}
     if world == 1:
-        line = bench_2d(args, torch, fb, cuda, shape, tape, bc, stream, flush, dev, peak, peak_src, sync_all)
+        line = bench_2d(args, torch, fb, cuda, shape, tape, bc, stream, flush, dev, peak, peak_src, sync_all, outputs)
         if not args.no_volume:
-            _, ms3, st3 = volume_on_one_gpu(torch, fb, cuda, shape, stream, flush)
+            img3, ms3, st3 = volume_on_one_gpu(torch, fb, cuda, shape, stream, flush)
+            if args.dump_outputs:
+                outputs.update(volume3d_outputs(img3))
             line["strong_scaling_base"] = {
                 "workload": f"models/{MODEL} 3D render {SIZE}^3 (the N > 1 workload), whole volume on 1 GPU",
                 "value": SIZE ** 3 / (ms3 * 1e-3) / 1e6, "unit": "Mvoxels/s", "ms_per_step": ms3,
                 "kernel_launches_per_step": int(st3["kernel_launches"])}
         if not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
         return
 
@@ -336,6 +393,8 @@ def main():
     with ClockSampler(local) as clocks:
         ms_local = time_steps(torch, stream, flush, step, args.steps, sync_all)
     cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        outputs.update(volume3d_outputs(image))   # the assembled frame, before the census render below reuses `image`
     ms_per_step = maxrank(ms_local)
     value = SIZE ** 3 / (ms_per_step * 1e-3) / 1e6
 
@@ -396,12 +455,14 @@ def main():
                          "rank0_stage_ms": {"interval_levels": [float(x) for x in stage[:5]], "k_voxels_3d": float(stage[9]),
                                             "k_normals_3d": float(stage[10])}},
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     dist.barrier()
     dist.destroy_process_group()
 
 
-def bench_2d(args, torch, fb, cuda, shape, tape, bc, stream, flush, dev, peak, peak_src, sync_all):
+def bench_2d(args, torch, fb, cuda, shape, tape, bc, stream, flush, dev, peak, peak_src, sync_all, outputs):
     cfg = fb.RenderConfig2D(SIZE, SIZE)
     image = torch.zeros((SIZE, SIZE), dtype=torch.float32, device=dev)
 
@@ -415,6 +476,8 @@ def bench_2d(args, torch, fb, cuda, shape, tape, bc, stream, flush, dev, peak, p
     with ClockSampler(dev.index or 0) as clocks:
         ms_per_step = time_steps(torch, stream, flush, step, args.steps, sync_all)
     cuda.synchronize()
+    if args.dump_outputs:
+        outputs.update(frame2d_outputs(image))    # before the per-kernel timing below renders into `image` again
     value = SIZE * SIZE / (ms_per_step * 1e-3) / 1e6
 
     # ---- per-kernel timing of one step (CUDA events inside the library, on the launching stream) ----
